@@ -1,7 +1,9 @@
 #!/usr/bin/env python
-"""bench.py — driver contract: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]`.
+"""bench.py — `python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]`.
 
-Prints ONE JSON line (rank 0).  A "step" = one pass of the hot path over one batch of synthetic images per GPU.
+Prints ONE JSON line (rank 0).  A "step" = one pass of the hot path over one batch of synthetic images per GPU; the
+resident and e2e loops of every workload, sub-benchmarks included, time K steps.  `--dump-outputs DIR` writes what the last timed step of the selected workload returned (rank 0)
+as DIR/<name>.npy: the same seeded inputs on every run, so two builds can be compared output for output.
 
 Workloads (BASELINE.json configs):
   depth_beit512     dpt_beit_large_512 @512x512, batch 32/GPU, depth only            (configs[1], the default once built)
@@ -106,6 +108,7 @@ class Stereo2048:
     dtype = "f64"  # the stereo / normal-map arithmetic type (fp64, truncating to u8); normalise is f32
     fill = "polylines_sharp"
     launches_per_step = 3 + 3 + 1  # normalise (init, minmax, quantise) + stereo (init, minmax, row) + normal map
+    outputs = ("depth", "stereo_sbs", "normal")
 
     def __init__(self, dev, rank):
         import torch
@@ -243,6 +246,24 @@ class GraphedStep:
         return self.outs
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, names, outs):
+    """Writes one step's outputs (CUDA tensors) as <dirname>/<name>.npy in float32 (float64 stays float64), 64 MB at most
+    in all: an output larger than its even share of that is written as its values at a fixed, seeded sample of its
+    flattened positions (the same positions on every run)."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(outs) - 4096                    # room for each file's .npy header
+    for name, o in zip(names, outs):
+        a = o.detach().cpu().numpy()
+        dt = np.float64 if a.dtype == np.float64 else np.float32
+        k = share // np.dtype(dt).itemsize
+        if a.size > k:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(os.path.join(dirname, f"{name}.npy"), a.astype(dt))
+
+
 WORKLOADS = {"stereo2048": Stereo2048}
 try:
     from bench_models import MODEL_WORKLOADS  # depth-network workloads, added once the tensor-core path is built
@@ -349,12 +370,14 @@ class Gatherer:
         torch.cuda.current_stream().wait_stream(self.side)
 
 
-def measure(wl, args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, with_funnel):
-    """One workload: resident-input throughput, dominant-kernel roofline, host-buffer e2e (+ funnel e2e, CPU baseline)."""
+def measure(wl, args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, with_funnel, dump_dir=None):
+    """One workload: resident-input throughput, dominant-kernel roofline, host-buffer e2e (+ funnel e2e, CPU baseline).
+    With `dump_dir`, rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     import torch
     import torch.distributed as dist
+    dump = (lambda outs: dump_outputs(dump_dir, wl.outputs, outs)) if (dump_dir and rank == 0) else None
     if hasattr(wl, "measure"):       # a workload with its own step structure (BOOST: one image, patch-parallel, strong scaling)
-        return wl.measure(args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, ClockSampler)
+        return wl.measure(args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, ClockSampler, dump)
     graphed = None
     if not args.no_graph:
         graphed = GraphedStep(lambda: wl.step_resident(False))
@@ -380,7 +403,7 @@ def measure(wl, args, world, dev, rank, local_rank, peaks, steps, with_cpu_basel
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        full_step(time_kernel=False)
+        outs = full_step(time_kernel=False)
     if gatherer is not None:
         gatherer.drain()
     e1.record()
@@ -388,6 +411,8 @@ def measure(wl, args, world, dev, rank, local_rank, peaks, steps, with_cpu_basel
     if world > 1:
         dist.barrier()
     clocks = sampler.stop() if sampler else None
+    if dump is not None:
+        dump(outs)
     ms_total = e0.elapsed_time(e1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -476,7 +501,10 @@ def main():
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-benchmarks (stereo2048, dav2_stereo) of the default run")
     ap.add_argument("--no-funnel", action="store_true", help="skip the core_generation_funnel (PIL in / PIL out) end-to-end measurement")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of --workload to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -503,7 +531,8 @@ def main():
         dist.barrier()
     peaks = _peaks()
     wl = WORKLOADS[args.workload](dev, rank)
-    line = measure(wl, args, world, dev, rank, local_rank, peaks, args.steps, not args.no_cpu_baseline, not args.no_funnel)
+    line = measure(wl, args, world, dev, rank, local_rank, peaks, args.steps, not args.no_cpu_baseline, not args.no_funnel,
+                   args.dump_outputs)
     if rank == 0 and world == 1 and not args.no_sub:
         subs = []
         for name in SUB_WORKLOADS.get(args.workload, []):
@@ -513,7 +542,7 @@ def main():
             torch.cuda.empty_cache()
             try:
                 wl = WORKLOADS[name](dev, rank)
-                sub = measure(wl, args, world, dev, rank, local_rank, peaks, max(2, min(args.steps, 5)), not args.no_cpu_baseline, False)
+                sub = measure(wl, args, world, dev, rank, local_rank, peaks, args.steps, not args.no_cpu_baseline, False)
                 sub["workload"] = name
                 subs.append(sub)
             except Exception as e:  # noqa: BLE001

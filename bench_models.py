@@ -113,6 +113,7 @@ class Dav2Stereo(_NetWorkload):
     B = 64
     dtype = "fp16"  # tensor-core operands fp16, fp32 accumulate / residual stream (the reference's GPU path is .half())
     fill = "polylines_sharp"
+    outputs = ("depth", "stereo_sbs", "normal")
     FLOP_PER_IMAGE = 1304.2e9  # SURVEY §8d, cross-checked there against FlopCounterMode on the reference module
     MODEL_TYPE = 14
     ATTN_KERNEL = "attention_fwd4_kernel<0> (fused softmax(QK^T)V, tcgen05 + TMEM, N = 1370, 16 heads x 64)"
@@ -205,6 +206,7 @@ class DepthBeit512(_NetWorkload):
     H = W = 512
     B = 32
     dtype = "fp16"
+    outputs = ("depth",)
     FLOP_PER_IMAGE = 962.7e9  # SURVEY §8d
     MODEL_TYPE = 1
     ATTN_KERNEL = "attention_fwd4_kernel<3> (fused softmax(QK^T + rel-pos bias)V, tcgen05 + TMEM, N = 1025, 16 heads x 64; + class-row kernel)"
@@ -289,6 +291,7 @@ class ZoeAnaglyph(_NetWorkload):
     B = 32
     dtype = "fp16"
     NET_W, NET_H = 384, 512
+    outputs = ("depth", "anaglyph")
     FLOP_PER_IMAGE = 2 * 962.7e9 + 2 * 10e9      # SURVEY 8d: two core forwards at 512x512 + the metric head (~1%)
     ATTN_KERNEL = "attention_fwd4_kernel<3> (fused softmax(QK^T + rel-pos bias)V of the BEiT-L-384 core at a 32x32 window, 64 forwards)"
     FC1_KERNEL = "gemm_tcgen05_2sm_kernel (block MLP fc1: M=64*1025, N=4096, K=1024, GELU epilogue)"
@@ -391,6 +394,7 @@ class BoostRes101:
     B = 1
     dtype = "fp16 (LeReS operands) / split fp16 = fp32-class (merge net), fp32 accumulate"
     RMAX = 1600                                   # the reference's default boost_rmax (src/backbone.py:36-49)
+    outputs = ("depth",)
 
     def __init__(self, dev, rank):
         from bench import make_images
@@ -412,7 +416,7 @@ class BoostRes101:
                 "height": self.H, "width": self.W, "boost_rmax": self.RMAX, "weights": "seeded synthetic, res101.pth / latest_net_G.pth layouts",
                 "l2_policy": "per-image activations (several GB) far exceed the 126 MB L2"}
 
-    def measure(self, args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, ClockSampler):
+    def measure(self, args, world, dev, rank, local_rank, peaks, steps, with_cpu_baseline, ClockSampler, dump=None):
         import torch
         import torch.distributed as dist
         from PIL import Image
@@ -432,12 +436,14 @@ class BoostRes101:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            self.pipe.run(self.rgb, self.RMAX, group=group, precomputed=plan, to_host=False)
+            depth = self.pipe.run(self.rgb, self.RMAX, group=group, precomputed=plan, to_host=False)
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
             dist.barrier()
         clocks = sampler.stop() if sampler else None
+        if dump is not None:
+            dump((depth,))
         launches = self.pipe.launches + self.pipe.depth.ops.launches + self.pipe.merge.ops.launches - n0
         t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:

@@ -1,393 +1,219 @@
-"""CPU, build container only: pins the oracle to the REAL reference imported from /root/reference.
-
-Skipped where the reference tree is absent (the GPU box); there the committed goldens carry the pin."""
+"""CPU: pins the oracle to the original extension's own code.  Every case recomputes through oracle/ what the original's
+functions and modules computed on the same seeded inputs, as recorded in tests/golden/oracle_pin_golden.npz by
+tests/golden/make_pin_golden.py (which runs the original).  Exact outputs are compared through their SHA-256; outputs
+compared within a tolerance of more than golden.make_pin_golden.SAMPLE values at a fixed, seeded sample of positions."""
+import os
 import warnings
 
 import numpy as np
 import pytest
 
+from golden import make_pin_golden as mk
 from oracle import normalmap as onm
-from oracle import ref_loader
 from oracle import stereo as ost
-from synth import noise_depth_u16, noise_rgb, synth_depth_u16, synth_rgb
-
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
+from synth import synth_rgb
 
 
 @pytest.fixture(scope="module")
-def ref():
+def gold():
     warnings.filterwarnings("ignore")
-    return ref_loader.stereo_module(), ref_loader.normalmap_module()
+    return np.load(os.path.join(os.path.dirname(__file__), "golden", "oracle_pin_golden.npz"))
 
 
-@pytest.mark.parametrize("fill", ['none', 'naive', 'naive_interpolating', 'polylines_soft', 'polylines_sharp'])
-def test_stereo_oracle_equals_reference(ref, fill):
-    rs, _ = ref
-    rng = np.random.default_rng(11)
-    for (h, w, seed, kind) in [(21, 67, 10, 'smooth'), (16, 50, 11, 'noise')]:
-        img = synth_rgb(h, w, seed) if kind == 'smooth' else noise_rgb(h, w, seed)
-        dep = synth_depth_u16(h, w, seed) if kind == 'smooth' else noise_depth_u16(h, w, seed)
-        for _ in range(3):
-            div, sep = float(rng.uniform(0.05, 15)), float(rng.uniform(-5, 5))
-            bal, ex = float(rng.uniform(-1, 1)), float(rng.choice([1.0, 2.0]))
-            a = rs.create_stereoimages(img, dep, div, sep, ['left-right', 'red-cyan-anaglyph'], bal, ex, fill)
-            b = ost.create_stereoimages(img, dep, div, sep, ['left-right', 'red-cyan-anaglyph'], bal, ex, fill)
-            for x, y in zip(a, b):
-                assert np.array_equal(np.asarray(x), np.asarray(y)), (fill, div, sep, bal, ex)
+@pytest.fixture(autouse=True)
+def _recorded_thread_count():
+    """the outputs were recorded with mk.THREADS torch threads, which keeps fp32 reductions in the same order here"""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(mk.THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
-def test_stereo_oracle_float_depth_equals_reference(ref):
-    rs, _ = ref
-    img = noise_rgb(12, 40, 5)
-    dep = np.random.default_rng(5).random((12, 40)).astype(np.float32)
+def _exact(gold, key, got):
+    assert mk.digest(got) == str(gold[key]), key
+
+
+def _close(gold, key, got, rel=None, abs_=None):
+    """`got` has the recorded output's shape and is within rel * max|output| (or abs_) of it at every stored position;
+    returns max|output|"""
+    got = np.asarray(got)
+    assert got.shape == tuple(gold[key + "_shape"]), key
+    scale = float(gold[key + "_absmax"])
+    err = float(np.abs(mk.sample(got).astype(np.float64) - gold[key].astype(np.float64)).max())
+    assert err <= (abs_ if abs_ is not None else rel * scale), (key, err, scale)
+    return scale
+
+
+@pytest.mark.parametrize("fill", mk.STEREO_FILLS)
+def test_stereo_oracle_equals_reference(gold, fill):
+    for ci, (img, dep, div, sep, bal, ex) in enumerate(mk.stereo_cases()):
+        b = ost.create_stereoimages(img, dep, div, sep, mk.STEREO_MODES, bal, ex, fill)
+        assert len(b) == len(mk.STEREO_MODES)
+        for m, y in zip(mk.STEREO_MODES, b):
+            _exact(gold, f"stereo_{fill}_{ci}_{m}", np.asarray(y))
+
+
+def test_stereo_oracle_float_depth_equals_reference(gold):
+    img, dep = mk.stereo_float_depth_case()
     for fill in ['naive', 'polylines_sharp']:
-        a = rs.create_stereoimages(img, dep, 3.0, fill_technique=fill)[0]
-        b = ost.create_stereoimages(img, dep, 3.0, fill_technique=fill)[0]
-        assert np.array_equal(np.asarray(a), np.asarray(b))
+        _exact(gold, f"stereo_float_{fill}", np.asarray(ost.create_stereoimages(img, dep, 3.0, fill_technique=fill)[0]))
 
 
-def test_normalmap_oracle_equals_reference(ref):
-    _, rn = ref
+def test_normalmap_oracle_equals_reference(gold):
     for seed in range(3):
-        dep = synth_depth_u16(30, 41, seed) if seed else noise_depth_u16(30, 41, seed)
-        for (pb, sb, qb, inv) in [(None, 3, None, False), (None, 5, None, True), (None, None, None, False),
-                                  (3, 3, 3, False), (None, 11, None, False), (9, 3, None, True), (None, 3, 11, False),
-                                  (None, 31, None, False), (31, 3, 31, False)]:
-            a = np.asarray(rn.create_normalmap(dep, pb, sb, qb, inv))
-            b = onm.create_normalmap(dep, pb, sb, qb, inv, return_array=True)
-            assert np.array_equal(a, b), (seed, pb, sb, qb, inv)
+        for ci, (pb, sb, qb, inv) in enumerate(mk.NORMAL_CASES):
+            _exact(gold, f"normal_{seed}_{ci}", onm.create_normalmap(mk.normal_depth(seed), pb, sb, qb, inv, return_array=True))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# D7 (round-2 row): the ZoeDepth-NK metric head oracle against the reference module built around a stub core
+# D7 (round-2 row): the ZoeDepth-NK metric head oracle against the original module built around a stub core
 # ---------------------------------------------------------------------------------------------------------------------
-def _zoedepth_reference_head(seed, base_hw):
-    import torch
-    import torch.nn as nn
-    ref_loader.bootstrap()
-    from dzoedepth.models.zoedepth_nk.zoedepth_nk_v1 import ZoeDepthNK
-    from oracle import zoedepth as ozd
-    g = torch.Generator().manual_seed(seed)
-    h, w = base_hw
-    shapes = [(32, 16 * h, 16 * w), (256, h, w), (256, 2 * h, 2 * w), (256, 4 * h, 4 * w), (256, 8 * h, 8 * w), (256, 16 * h, 16 * w)]
-    feats = [torch.randn(2, c, hh, ww, generator=g) * 0.7 for c, hh, ww in shapes]
-    feats[0] = feats[0].abs()                      # out_conv is a post-ReLU activation in the core
-
-    class StubCore(nn.Module):                     # hands the head fixed activations (MidasCore.forward, midas.py:258-276)
-        output_channels = (256, 256, 256, 256, 256)
-
-        def forward(self, x, denorm=False, return_rel_depth=False):
-            return torch.zeros(x.shape[0], x.shape[2], x.shape[3]), [f.clone() for f in feats]
-
-    cfg = {k: ozd.CONFIG[k] for k in ("bin_embedding_dim", "n_attractors", "attractor_alpha", "attractor_gamma", "min_temp", "max_temp")}
-
-    class AttrDict(dict):                          # the reference reads its config entries as attributes (EasyDict)
-        __getattr__ = dict.__getitem__
-
-    model = ZoeDepthNK(StubCore(), bin_conf=[AttrDict(c) for c in ozd.CONFIG["bin_conf"]], bin_centers_type="softplus", attractor_kind="mean",
-                       attractor_type="inv", memory_efficient=True, **cfg).eval()
-    with torch.no_grad():                          # seeded weights with enough spread to exercise every branch
-        for name, p in model.named_parameters():
-            p.copy_(torch.randn(p.shape, generator=g) * (0.05 if p.ndim > 1 else 0.02))
-            if name.endswith("norm1.weight") or name.endswith("norm2.weight"):
-                p.add_(1.0)
-    sd = {k: v.detach().clone() for k, v in model.state_dict().items() if not k.startswith("core.")}
-    return model, feats, sd
+def _zoedepth_head(gold, seed, base_hw):
+    lay = mk.layout(gold, "zoe_head")
+    buffers = {k[len("zoe_buffer_"):]: gold[k] for k in gold.files if k.startswith("zoe_buffer_")}
+    return mk.zoe_head_inputs(seed, base_hw, lay, buffers)
 
 
-@pytest.mark.parametrize("seed,base_hw", [(0, (3, 4)), (1, (4, 3)), (2, (2, 2))])
-def test_zoedepth_head_oracle_equals_reference(seed, base_hw):
+@pytest.mark.parametrize("seed,base_hw", mk.ZOE_HEADS)
+def test_zoedepth_head_oracle_equals_reference(gold, seed, base_hw):
     import torch
     from oracle import zoedepth as ozd
-    model, feats, sd = _zoedepth_reference_head(seed, base_hw)
+    feats, sd = _zoedepth_head(gold, seed, base_hw)
     with torch.no_grad():
-        want = model(torch.zeros(2, 3, feats[0].shape[2], feats[0].shape[3]))
         got_depth, got_logits, name = ozd.metric_head(feats, sd)
-    assert torch.equal(got_logits, want["domain_logits"]) or (got_logits - want["domain_logits"]).abs().max() < 1e-5
-    err = (got_depth - want["metric_depth"]).abs().max().item()
-    assert err <= 1e-5 * want["metric_depth"].abs().max().item(), (name, err)
+    _close(gold, f"zoe_head_{seed}_logits", got_logits.numpy(), abs_=1e-5)
+    _close(gold, f"zoe_head_{seed}_depth", got_depth.numpy(), rel=1e-5)
 
 
-@pytest.mark.parametrize("pad,flip", [(True, True), (True, False), (False, True)])
-def test_zoedepth_tta_wrapper_equals_reference(pad, flip):
+@pytest.mark.parametrize("pad,flip", mk.ZOE_TTA)
+def test_zoedepth_tta_wrapper_equals_reference(gold, pad, flip):
     """DepthModel.infer (pad + flip augmentation) around the same head: the stub core ignores its input, so this pins the
     padding arithmetic, the bicubic resize back to the padded size, the crop and the flip average."""
     import torch
     from oracle import zoedepth as ozd
-    model, feats, sd = _zoedepth_reference_head(3, (2, 3))
-    x = torch.rand(2, 3, 40, 56, generator=torch.Generator().manual_seed(5))
+    feats, sd = _zoedepth_head(gold, 3, (2, 3))
     with torch.no_grad():
-        want = model.infer(x, pad_input=pad, with_flip_aug=flip)
-        got = ozd.infer(lambda t: ozd.metric_head(feats, sd)[0], x, pad_input=pad, with_flip_aug=flip)
-    assert got.shape == want.shape == (2, 1, 40, 56)
-    assert (got - want).abs().max().item() <= 1e-5 * want.abs().max().item()
+        got = ozd.infer(lambda t: ozd.metric_head(feats, sd)[0], mk.zoe_tta_input(), pad_input=pad, with_flip_aug=flip)
+    assert got.shape == (2, 1, 40, 56)
+    _close(gold, f"zoe_tta_{int(pad)}{int(flip)}", got.numpy(), rel=1e-5)
 
 
-@pytest.mark.parametrize("smoothening", ["none", "experimental", "something-else"])
-def test_video_normalisation_equals_reference(smoothening):
+@pytest.mark.parametrize("smoothening", mk.VIDEO_SMOOTHENING)
+def test_video_normalisation_equals_reference(gold, smoothening):
     """§8(f) rank 1 groundwork: cross-frame normalisation of video mode (src/video_mode.py:103-128)."""
-    ref_loader.bootstrap()
-    try:
-        from src import video_mode
-    except Exception as e:          # optional host dependencies of the video writer
-        pytest.skip(f"src.video_mode not importable here: {e}")
     from oracle import video as ovid
-    rng = np.random.default_rng(11)
-    frames = [(rng.standard_normal((24, 32)) * (1 + 0.3 * i) + 0.1 * i).astype(np.float32) for i in range(7)]
-    want = video_mode.process_predicitons([f.copy() for f in frames], smoothening)
-    got = ovid.process_predictions([f.copy() for f in frames], smoothening)
-    assert len(got) == len(want)
-    for g, w in zip(got, want):
-        assert g.dtype == w.dtype and np.array_equal(g, w)
+    got = ovid.process_predictions(mk.video_frames(), smoothening)
+    assert len(got) == int(gold[f"video_{smoothening}_count"])
+    for i, g in enumerate(got):
+        _exact(gold, f"video_{smoothening}_{i}", g)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# D8 (round-2 row): LeReS ResNeXt-101 32x8d + decoder oracle against the reference module with the same state_dict
+# D8 (round-2 row): LeReS ResNeXt-101 32x8d + decoder oracle against the original module with the same state_dict
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
-def leres_reference():
-    import torch
-    ref_loader.bootstrap()
-    from lib.multi_depth_model_woauxi import RelDepthModel
-    model = RelDepthModel(backbone="resnext101").eval()
-    g = torch.Generator().manual_seed(21)
-    with torch.no_grad():                     # seeded weights / running statistics that keep activations O(1) through 100+ layers
-        for name, p in model.named_parameters():
-            if p.ndim == 4:
-                fan_in = p.shape[1] * p.shape[2] * p.shape[3]
-                p.copy_(torch.randn(p.shape, generator=g) * (1.0 / fan_in ** 0.5))
-            elif name.endswith(".weight"):
-                p.copy_((0.3 if "bn3" in name else 1.0) + 0.05 * torch.randn(p.shape, generator=g))
-            else:
-                p.copy_(0.05 * torch.randn(p.shape, generator=g))
-        for name, b in model.named_buffers():
-            if name.endswith("running_mean"):
-                b.copy_(0.1 * torch.randn(b.shape, generator=g))
-            elif name.endswith("running_var"):
-                b.copy_(0.5 + torch.rand(b.shape, generator=g))
-    return model, {k: v.detach().clone() for k, v in model.state_dict().items()}
+def leres_weights(gold):
+    return mk.leres_weights(mk.layout(gold, "leres"))
 
 
-def test_leres_synthetic_state_dict_matches_reference_module():
-    """oracle.synth_weights.make_leres_state_dict has exactly the reference module's keys and shapes (strict load, only the
-    BatchNorm step counters are left out) and the oracle reproduces the reference module with it."""
+def test_leres_synthetic_state_dict_matches_reference_module(gold):
+    """oracle.synth_weights.make_leres_state_dict has exactly the original module's keys and shapes (strict load, only the
+    BatchNorm step counters are left out) and the oracle reproduces the original module with it."""
     import torch
-    ref_loader.bootstrap()
-    from lib.multi_depth_model_woauxi import RelDepthModel
     from oracle import leres, synth_weights
     sd = synth_weights.make_leres_state_dict(seed=2)
-    model = RelDepthModel(backbone="resnext101").eval()
-    res = model.load_state_dict(sd, strict=False)
-    assert not res.unexpected_keys and all(k.endswith("num_batches_tracked") for k in res.missing_keys)
-    x = torch.randn(1, 3, 64, 96, generator=torch.Generator().manual_seed(4))
+    want = {name: shape for name, shape, _ in mk.layout(gold, "leres")}
+    assert set(sd) <= set(want) and all(k.endswith("num_batches_tracked") for k in set(want) - set(sd))
+    assert all(list(v.shape) == want[k] for k, v in sd.items())
     with torch.no_grad():
-        want = model.depth_model(x)
-        got = leres.forward(sd, x)
-    assert torch.isfinite(want).all() and want.abs().max().item() > 1e-3
-    assert (got - want).abs().max().item() <= 1e-5 * want.abs().max().item()
+        got = leres.forward(sd, mk.leres_synth_input())
+    assert _close(gold, "leres_synth", got.numpy(), rel=1e-5) > 1e-3
 
 
-def test_leres_network_oracle_equals_reference(leres_reference):
+def test_leres_network_oracle_equals_reference(gold, leres_weights):
     import torch
     from oracle import leres
-    model, sd = leres_reference
-    x = torch.randn(1, 3, 96, 128, generator=torch.Generator().manual_seed(4))
     with torch.no_grad():
-        want = model.depth_model(x)
-        got = leres.forward(sd, x)
-    assert got.shape == want.shape == (1, 1, 96, 128)
-    scale = want.abs().max().item()
-    assert scale > 0 and torch.isfinite(want).all()
-    assert (got - want).abs().max().item() <= 1e-5 * scale
+        got = leres.forward(leres_weights, mk.leres_network_input())
+    assert got.shape == (1, 1, 96, 128)
+    assert _close(gold, "leres_network", got.numpy(), rel=1e-5) > 0
 
 
-def test_leres_estimate_equals_reference(leres_reference):
+def test_leres_estimate_equals_reference(gold, leres_weights):
     """estimateleres (BGR flip, cv2 resize, scale_torch, cubic resize back) around the same network."""
-    import torch
     from oracle import leres
-    model, sd = leres_reference
-    try:
-        from src import depthmap_generation as dg
-    except Exception as e:
-        pytest.skip(f"src.depthmap_generation not importable here: {e}")
-    dg.depthmap_device = torch.device("cpu")
-    import cv2
     rgb = synth_rgb(70, 90, 3)
-    img = cv2.cvtColor(rgb, cv2.COLOR_BGR2RGB) / 255.0       # what ModelHolder.get_raw_prediction hands over (:381)
-    want = dg.estimateleres(img, model, 64, 96)
-    got, invert = leres.get_raw_prediction(rgb, sd, 64, 96)
-    assert invert is True and got.shape == want.shape == (70, 90)
-    assert np.abs(got - want).max() <= 1e-5 * np.abs(want).max()
-    want = dg.estimateleres(rgb, model, 96, 64)               # and the function itself on a uint8 array
-    got = leres.estimateleres(rgb, sd, 96, 64)
-    assert np.abs(got - want).max() <= 1e-5 * np.abs(want).max()
+    got, invert = leres.get_raw_prediction(rgb, leres_weights, 64, 96)
+    assert invert is True and got.shape == (70, 90)
+    _close(gold, "leres_estimate_img", got, rel=1e-5)
+    _close(gold, "leres_estimate_u8", leres.estimateleres(rgb, leres_weights, 96, 64), rel=1e-5)
 
 
-def test_pix2pix_unet_oracle_equals_reference():
+def test_pix2pix_unet_oracle_equals_reference(gold):
     """D9 groundwork: the BOOST merge network (10-level U-Net, norm 'none') and its input preparation."""
     import torch
-    ref_loader.bootstrap()
-    from pix2pix.models import networks
     from oracle import pix2pix as op2p
-    net = networks.define_G(2, 1, 64, 'unet_1024', 'none', False, 'normal', 0.02, []).eval()
-    g = torch.Generator().manual_seed(31)
-    with torch.no_grad():
-        for name, p in net.named_parameters():
-            if p.ndim == 4:
-                p.copy_(torch.randn(p.shape, generator=g) * (1.6 / (p.shape[1] * 16) ** 0.5))
-            else:
-                p.copy_(0.05 * torch.randn(p.shape, generator=g))
-    sd = {k: v.detach().clone() for k, v in net.state_dict().items()}
-    rng = np.random.default_rng(5)
-    outer = rng.standard_normal((1024, 1024)).astype(np.float32)
-    inner = (outer * 0.5 + rng.standard_normal((1024, 1024)).astype(np.float32)).astype(np.float32)
-    x = op2p.merge_input(outer, inner)
+    sd = mk.pix2pix_weights(mk.layout(gold, "pix2pix"))
+    x = mk.pix2pix_input()
     assert x.shape == (1, 2, 1024, 1024) and float(x.min()) == -1.0 and float(x.max()) == 1.0
     with torch.no_grad():
-        want = net(x.clone())
         got = op2p.unet(sd, x.clone())
-    assert got.shape == want.shape == (1, 1, 1024, 1024)
-    assert float(want.abs().max()) > 1e-3          # the seeded weights keep a signal through the 20 layers
-    assert (got - want).abs().max().item() <= 1e-5
+    assert got.shape == (1, 1, 1024, 1024)
+    assert _close(gold, "pix2pix_unet", got.numpy(), abs_=1e-5) > 1e-3     # the seeded weights keep a signal through the 20 layers
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# Depth-Anything-V2 (D5 / D6): the oracle restatement against the reference's own DepthAnythingV2 module
+# Depth-Anything-V2 (D5 / D6): the oracle restatement against the original's own DepthAnythingV2 module
 # ---------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("encoder,hw,net", [("vits", (70, 98), 70), ("vits", (84, 56), 56), ("vitb", (70, 70), 70)])
-def test_dav2_oracle_equals_reference(encoder, hw, net):
-    """ddepth_anything_v2/depth_anything_v2/dpt.py:176-221 + src/depthmap_generation.py:375-403,548-559: strict
-    state_dict load of the synthetic weights into the reference module, then the reference's own pre-processing /
-    forward / final resize against oracle.dav2.get_raw_prediction on the same uint8 image -> identical floats."""
-    import cv2
-    import torch
-    import torch.nn.functional as F
+@pytest.mark.parametrize("encoder,hw,net", mk.DAV2_CASES)
+def test_dav2_oracle_equals_reference(gold, encoder, hw, net):
+    """ddepth_anything_v2/depth_anything_v2/dpt.py:176-221 + src/depthmap_generation.py:375-403,548-559: the synthetic
+    weights have exactly the original module's keys and shapes (it loads them strictly), and its own pre-processing /
+    forward / final resize on them matches oracle.dav2.get_raw_prediction on the same uint8 image."""
     from oracle import dav2 as odav2
     from oracle import synth_weights
-    cls = ref_loader.dav2_class()
     sd = synth_weights.make_dav2_state_dict(encoder, seed=1)
-    cfg = odav2.CONFIGS[encoder]
-    model = cls(encoder=encoder, features=cfg['features'], out_channels=cfg['out_channels']).eval()
-    missing = model.load_state_dict(sd, strict=True)
-    assert not missing.missing_keys and not missing.unexpected_keys
-    rgb = synth_rgb(hw[0], hw[1], 3)
-    # the reference's call chain, verbatim: get_raw_prediction (:381) -> estimatedepthanything_v2 (:548-559)
-    img = cv2.cvtColor(np.asarray(rgb), cv2.COLOR_BGR2RGB) / 255.0
-    with torch.no_grad():
-        image = cv2.cvtColor((img * 255.1).astype('uint8'), cv2.COLOR_BGR2RGB)
-        image, (h, w) = model.image2tensor(image, net)
-        image = image.to('cpu')
-        depth = model.forward(image)
-        depth = F.interpolate(depth[:, None], (h, w), mode="bilinear", align_corners=True)[0, 0]
-    want = depth.cpu().numpy()
-    got, invert = odav2.get_raw_prediction(rgb, sd, encoder, net)
+    assert {k: list(v.shape) for k, v in sd.items()} == {name: shape for name, shape, _ in mk.layout(gold, "dav2_" + encoder)}
+    got, invert = odav2.get_raw_prediction(synth_rgb(hw[0], hw[1], 3), sd, encoder, net)
     assert invert is False
-    assert want.max() - want.min() > 0.1          # a non-degenerate map (default init would be identically zero)
-    assert got.shape == want.shape == tuple(hw)
-    assert float(np.abs(got - want).max()) <= 1e-6 * float(np.abs(want).max()), float(np.abs(got - want).max())
+    key = f"dav2_{encoder}_{hw[0]}x{hw[1]}_{net}"
+    assert got.shape == tuple(hw)
+    assert float(gold[key].max() - gold[key].min()) > 0.1      # a non-degenerate map (default init would be identically zero)
+    _close(gold, key, got, rel=1e-6)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# D9: the BOOST driver (resolution search, patch selection, double estimation, merge + blend) against the reference's own
+# D9: the BOOST driver (resolution search, patch selection, double estimation, merge + blend) against the original's own
 # functions.  The two networks are stand-ins (cheap, deterministic, the same on both sides): the real ones are pinned above.
 # ---------------------------------------------------------------------------------------------------------------------
-class _FakeLeres:
-    """stands for RelDepthModel: estimateleres calls model.depth_model(normalised [1,3,h,w])"""
-
-    @staticmethod
-    def depth_model(x):
-        import torch
-        import torch.nn.functional as F
-        g = x.mean(dim=1, keepdim=True)
-        return F.avg_pool2d(g, 9, 1, 4) + 0.25 * torch.sin(3.0 * x[:, :1]) + 0.1 * x[:, 2:3]
-
-
-class _FakePix2Pix:
-    """stands for Pix2Pix4DepthModel: set_input / test / get_current_visuals (pix2pix/models/pix2pix4depth_model.py:96-116)"""
-
-    def set_input(self, outer, inner):
-        from oracle import pix2pix as op2p
-        self.real_A = op2p.merge_input(outer, inner)
-
-    def test(self):
-        import torch
-        o, i = self.real_A[:, :1], self.real_A[:, 1:]
-        self.fake_B = torch.tanh(0.7 * o + 0.5 * i + 0.1 * o * i)
-
-    def get_current_visuals(self):
-        return {"fake_B": self.fake_B}
-
-
-def _boost_reference_module():
-    import torch
-    ref_loader.bootstrap()
-    try:
-        from src import depthmap_generation as dg
-    except Exception as e:
-        pytest.skip(f"src.depthmap_generation not importable here: {e}")
-    dg.depthmap_device = torch.device("cpu")
-    import skimage.measure as sm
-    from oracle import boost
-    sm.block_reduce = lambda img, block, func: boost.block_reduce_max(img, block[0])   # skimage is absent here (SURVEY A.5); zero-padded max pool
-    dg.skimage = __import__("skimage")
-    return dg
-
-
-def _fake_estimate(img, msize):
-    import cv2
-    from oracle import leres
-    with __import__("torch").no_grad():
-        pred = _FakeLeres.depth_model(leres.preprocess(img, msize, msize)).squeeze().numpy()
-    return cv2.resize(pred, (img.shape[1], img.shape[0]), interpolation=cv2.INTER_CUBIC)
-
-
-def _fake_merge(outer, inner):
-    p = _FakePix2Pix()
-    p.set_input(outer, inner)
-    p.test()
-    return p.fake_B.squeeze().numpy()
-
-
-@pytest.mark.parametrize("hw,rmax", [((300, 420), 1600), ((520, 360), 1200)])
-def test_boost_selection_equals_reference(hw, rmax):
+@pytest.mark.parametrize("hw,rmax", mk.BOOST_SELECTION)
+def test_boost_selection_equals_reference(gold, hw, rmax):
     """calculateprocessingres + generatepatchs + generatemask: integer / index results, compared exactly."""
-    import cv2
     from oracle import boost
-    dg = _boost_reference_module()
-    rgb = synth_rgb(hw[0], hw[1], 11)
-    img = cv2.cvtColor(rgb, cv2.COLOR_BGR2RGB) / 255.0
-    want = dg.calculateprocessingres(img, 448, 0.2, 3, rmax)
+    img = mk.boost_image(hw, 11)
     got = boost.calculateprocessingres(img, 448, 0.2, 3, rmax)
+    want = gold[f"boost_res_{hw[0]}x{hw[1]}"]
     assert got[0] == want[0] and got[1] == want[1]
-    factor = max(min(1, 4 * got[1] * got[0] / rmax), 0.2)
-    a, b = boost.target_size(img.shape, got[0], factor)
-    big = cv2.resize(img, (b, a), interpolation=cv2.INTER_CUBIC)
-    wantp = dg.generatepatchs(big, 896, factor)
+    big, factor = mk.boost_big_image(img, got, rmax)
     gotp = boost.generatepatchs(big, 896, factor)
+    wantp = gold[f"boost_rects_{hw[0]}x{hw[1]}"]
     assert len(gotp) == len(wantp) and len(gotp) > 0
-    assert [kv[1]["rect"] for kv in gotp] == [list(kv[1]["rect"]) for kv in wantp]
-    assert np.array_equal(boost.generatemask((300, 300)), dg.generatemask((300, 300)))
+    assert [list(kv[1]["rect"]) for kv in gotp] == wantp.tolist()
+    _exact(gold, "boost_mask", boost.generatemask((300, 300)))
 
 
-def test_boost_estimate_equals_reference():
+def test_boost_estimate_equals_reference(gold):
     """estimateboost end to end (model type 0: receptive field 448, patches at 896) with the stand-in networks."""
-    import cv2
     from oracle import boost
-    dg = _boost_reference_module()
-    rgb = synth_rgb(300, 420, 12)
-    img = cv2.cvtColor(rgb, cv2.COLOR_BGR2RGB) / 255.0
-    want = dg.estimateboost(img.copy(), _FakeLeres(), 0, _FakePix2Pix(), 1600)
     info = {}
-    got = boost.estimateboost(img.copy(), 0, _fake_estimate, _fake_merge, 1600, info=info)
-    assert got.shape == want.shape == (300, 420) and len(info["patches"]) >= 2
-    assert np.abs(got - want).max() <= 1e-6 * np.abs(want).max()
+    got = boost.estimateboost(mk.boost_image((300, 420), 12), 0, mk.fake_estimate, mk.fake_merge, 1600, info=info)
+    assert got.shape == (300, 420) and len(info["patches"]) >= 2
+    _close(gold, "boost_estimate", got, rel=1e-6)
 
 
-def test_pix2pix_synthetic_state_dict_matches_reference_module():
-    """oracle.synth_weights.make_pix2pix_state_dict loads strictly into the reference generator"""
-    ref_loader.bootstrap()
-    from pix2pix.models import networks
+def test_pix2pix_synthetic_state_dict_matches_reference_module(gold):
+    """oracle.synth_weights.make_pix2pix_state_dict loads strictly into the original generator"""
     from oracle import synth_weights
-    net = networks.define_G(2, 1, 64, 'unet_1024', 'none', False, 'normal', 0.02, [])
-    res = net.load_state_dict(synth_weights.make_pix2pix_state_dict(seed=1), strict=True)
-    assert not res.missing_keys and not res.unexpected_keys
+    sd = synth_weights.make_pix2pix_state_dict(seed=1)
+    assert {k: list(v.shape) for k, v in sd.items()} == {name: shape for name, shape, _ in mk.layout(gold, "pix2pix")}
