@@ -176,9 +176,10 @@ int dm_im2col_s2_f16(const void *in, int B, int H, int W, int C, void *out, void
 int dm_concat_readout_f16(const float *x, int B, int N, int C, void *out, void *stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
- * D7 — ZoeDepth-NK on top of the DPT-BEiT core (csrc/zoe_kernels.cu).   replaces
+ * D7 — ZoeDepth-NK / -N / -K on top of the DPT-BEiT core (csrc/zoe_kernels.cu).   replaces
  *   dzoedepth/models/depth_model.py:57-152 (pad + flip test-time augmentation), base_models/midas.py:175-186 (PrepForMidas),
  *   zoedepth_nk/zoedepth_nk_v1.py:159-243 (router, seed bins, attractors, conditional log-binomial),
+ *   zoedepth/zoedepth_v1.py:120-186 (single metric head), layers/localbins_layers.py:29-68 (normed seed bins),
  *   layers/attractor.py:127-208, layers/dist_layers.py:29-121, layers/patch_transformer.py:29-92.
  * Forward index f = 2*b + flip: image b and its horizontal flip go through the network as one batch of 2B forwards.
  * `logits` is fp32 [F, lld]: columns 0 / 1 are the router's nyu / kitti logits of that forward; every head kernel picks
@@ -201,12 +202,30 @@ int dm_resize_add_nhwc_f16(const void *a, const void *b_small, int B, int Hs, in
  * head*32; b_prev fp32 [F,Hp,Wp,64] is resized (bilinear, align_corners) to H x W; b_out fp32 [F,H,W,64] */
 int dm_zoe_attractor(const float *A, int lda, const float *logits, int lld, const float *b_prev, int F, int Hp, int Wp, int H, int W,
                      float *b_out, void *stream);
+/* Single-head attractor layer of ZoeDepth-N / -K (inverse attractor, mean over n_attractors in {16, 8, 4, 1}).  A fp32
+ * [F*H*W, lda], the layer's last 1x1 conv before its activation.  normed = 0 (AttractorLayerUnnormed): attractor i is
+ * softplus(A[:, i]).  normed = 1 (AttractorLayer): attractor i is relu(A[:, 2i]) + 1e-3; with B_sorted != NULL also
+ * B_sorted fp32 [F,H,W,64] = clip(sort_ascending((max - min) * b_out + min), min, max) per pixel.  b_prev / b_out as in
+ * dm_zoe_attractor (b_out is the normed b_new for normed = 1) */
+int dm_zoe_attractor_single(const float *A, int lda, int n_attractors, int normed, const float *b_prev, int F, int Hp, int Wp, int H, int W,
+                            float min_depth, float max_depth, float *b_out, float *B_sorted, void *stream);
+/* SeedBinRegressor's normed bin centres, rescaled to [0, 1] as ZoeDepth-K's first b_prev: per row r of seed fp32 [rows, ld]
+ * (64 used, before the final ReLU): w = relu(seed) + 1e-3 normalised to sum max - min, edges = cumsum([min, w]),
+ * out fp32 [rows, 64] = (midpoints of the edges - min) / (max - min) */
+int dm_zoe_seed_normed(const float *seed, int ld, long long rows, float min_depth, float max_depth, float *out, void *stream);
 /* ConditionalLogBinomial + expectation over the 64 bin centres, per net pixel.  o32: relu'd out_conv activation fp16
  * [F,nh,nw,ldo] (32 channels used); ze fp32 [F,h3,w3,ldz] = W_e . b_emb (head at column head*64, 40 used); bc fp32
  * [F,h3,w3,64] bin centres; wo [2][32][40], b0 [2][40], w2 [2][4][40], b2 [2][4] fp32 device arrays; out fp32 [F,nh,nw] */
 int dm_zoe_clb_final(const void *o32, int ldo, const float *ze, int ldz, const float *bc, const float *logits, int lld, const float *wo,
                      const float *b0, const float *w2, const float *b2, int F, int nh, int nw, int h3, int w3, float min_temp, float max_temp,
                      float *out, void *stream);
+/* dm_zoe_clb_final for the single metric head of ZoeDepth-N / -K: 161 inputs = out_conv (32) + relative depth (1) + bin
+ * embedding (128), 80 hidden units, no router.  The relative depth is relu(w_rel . out_conv + b_rel) (w_rel fp32 [32]: the
+ * core's last 1x1 conv).  ze fp32 [F,h3,w3,ldz]: W_e . b_emb at columns 0..79; wo [32][80], wr [80] (relative-depth column),
+ * b0 [80], w2 [4][80], b2 [4] fp32 device arrays */
+int dm_zoe_clb_final_single(const void *o32, int ldo, const float *ze, int ldz, const float *bc, const float *wo, const float *wr, const float *b0,
+                            const float *w2, const float *b2, const float *w_rel, float b_rel, int F, int nh, int nw, int h3, int w3,
+                            float min_temp, float max_temp, float *out, void *stream);
 /* out[b] = mean(crop(bicubic(d[2b])), unflip(crop(bicubic(d[2b+1])))): d fp32 [2B,nh,nw] -> out fp32 [B,H,W] */
 int dm_zoe_tta_combine(const float *d, int B, int nh, int nw, int pad_h, int pad_w, int H, int W, float *out, void *stream);
 

@@ -74,6 +74,7 @@ EXPORTS = [
     "dm_assemble_tokens", "dm_layernorm_f16", "dm_resize_bilinear_nhwc_f16", "dm_resize_f32", "dm_im2col_s2_f16", "dm_concat_readout_f16",
     "dm_zoe_preprocess_patchify", "dm_layernorm_post_f16", "dm_attention_small_f16", "dm_cast_f32_f16", "dm_zoe_select_softplus",
     "dm_resize_add_nhwc_f16", "dm_zoe_attractor", "dm_zoe_clb_final", "dm_zoe_tta_combine",
+    "dm_zoe_attractor_single", "dm_zoe_seed_normed", "dm_zoe_clb_final_single",
     "dm_video_workspace_bytes", "dm_video_blend", "dm_video_minmax", "dm_video_scale_f32", "dm_video_select_init", "dm_video_select_hist",
     "dm_video_select_pick", "dm_video_select_bounds", "dm_video_scale_f64",
     "dm_model_create", "dm_model_destroy", "dm_model_net_size", "dm_model_launches", "dm_depth_forward", "dm_dinov2_pos_embed", "dm_beit_rel_table", "dm_vit_pos_embed",
@@ -196,6 +197,10 @@ def _bind_optional(L):
         L.dm_zoe_attractor.argtypes = [vp, i32, vp, i32, vp, i32, i32, i32, i32, i32, vp, vp]
         L.dm_zoe_clb_final.argtypes = [vp, i32, vp, i32, vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, i32, f32, f32, vp, vp]
         L.dm_zoe_tta_combine.argtypes = [vp, i32, i32, i32, i32, i32, i32, i32, vp, vp]
+    if hasattr(L, "dm_zoe_clb_final_single"):
+        L.dm_zoe_attractor_single.argtypes = [vp, i32, i32, i32, vp, i32, i32, i32, i32, i32, f32, f32, vp, vp, vp]
+        L.dm_zoe_seed_normed.argtypes = [vp, i32, c.c_longlong, f32, f32, vp, vp]
+        L.dm_zoe_clb_final_single.argtypes = [vp, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, f32, i32, i32, i32, i32, i32, f32, f32, vp, vp]
 
 
 def check(rc: int, what: str = ""):

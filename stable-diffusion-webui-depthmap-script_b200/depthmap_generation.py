@@ -7,8 +7,8 @@
 the bench.  The network forward is a sequence of C-ABI calls (tcgen05 GEMM / implicit-GEMM conv / fused attention /
 LayerNorm / resize kernels, include/depthmap_b200.h); PyTorch only owns device memory and the stream.
 
-Implemented model types: 1, 2 (MiDaS 3.1 DPT-BEiT-L 512 / 384), 3 (MiDaS 3.0 DPT-Large 384), 9 (ZoeDepth-NK) and 12, 13, 14
-(Depth-Anything-V2 S/B/L).  Others raise NotImplementedError naming the type.
+Implemented model types: 0 (LeReS res101), 1, 2 (MiDaS 3.1 DPT-BEiT-L 512 / 384), 3 (MiDaS 3.0 DPT-Large 384), 7, 8, 9
+(ZoeDepth-N, -K, -NK) and 12, 13, 14 (Depth-Anything-V2 S/B/L).  Others raise NotImplementedError naming the type.
 Weights: a state_dict in the upstream checkpoint layout (``depth_anything_v2_vit{s,b,l}.pth``), packed once at load
 into the kernels' layout (fp16 GEMM operands, (ky,kx,cin)-ordered conv filters, ConvTranspose as GEMM + pixel shuffle).
 """
@@ -1070,12 +1070,13 @@ ZOE_CONFIG = dict(n_bins=64, emb=128, min_temp=0.0212, max_temp=50.0, router_dim
 
 
 class ZoeDepthNKEngine(DptBeitEngine):
-    """ZoeDepth-NK (model types 7-9 share this head family; 9 = zoedepth_nk) on the sm_100a kernels: DepthModel.infer_pil
+    """ZoeDepth-NK (model type 9 = zoedepth_nk) on the sm_100a kernels: DepthModel.infer_pil
     (pad + flip test-time augmentation, dzoedepth/models/depth_model.py:57-152), PrepForMidas (base_models/midas.py:175-186),
     the DPT-BEiT-L-384 core with MidasCore's hooks (midas.py:258-319) and the metric head of ZoeDepthNK.forward
     (zoedepth_nk/zoedepth_nk_v1.py:159-243).  Image b and its horizontal flip run as forwards 2b / 2b+1 of ONE batch; the
     router picks nyu / kitti per forward on the device (argmax of two logits, no host sync, no cross-image vote).
-    Checkpoint layout: MiDaS weights under "core.core.", head weights at the top level."""
+    Checkpoint layout: MiDaS weights under "core.core.", head weights at the top level.  ZoeDepthEngine (types 7 and 8)
+    shares everything but the head."""
 
     def __init__(self, state_dict, device, core_name='beitl16_384'):
         core_sd = {k[len("core.core."):]: v for k, v in state_dict.items() if k.startswith("core.core.")}
@@ -1085,25 +1086,35 @@ class ZoeDepthNKEngine(DptBeitEngine):
         self._zbuf_key, self._zbufs = None, {}
 
     # ---- weights -------------------------------------------------------------------------------------------------------
+    def _hw(self, sd, key, rows=None, cols=None):
+        """1x1 conv / linear weight -> fp16 [rows, cols] (zero padded)"""
+        import torch
+        t = sd[key + '.weight'].detach().to(self.device).float()
+        t = t.reshape(t.shape[0], -1)
+        r, c = rows or t.shape[0], cols or t.shape[1]
+        o = torch.zeros(r, c, dtype=torch.float16, device=self.device)
+        o[:t.shape[0], :t.shape[1]] = t.to(torch.float16)
+        return o
+
+    def _hb(self, sd, key, n=None):
+        """bias -> fp32 [n] (zero padded)"""
+        import torch
+        t = sd[key + '.bias'].detach().to(self.device).float().reshape(-1)
+        o = torch.zeros(n or t.numel(), dtype=torch.float32, device=self.device)
+        o[:t.numel()] = t
+        return o
+
+    def _pack_out_conv(self, z):
+        # out_conv with 64 output channels (32 real + 32 zero) so the stored activation is a valid GEMM-friendly NHWC tensor
+        z['oc2_w'] = _conv_w(self._oc2_weight.to(self.device), self.F2p, 32)
+        z['oc2_b'] = self._oc2_bias.to(self.device).float().contiguous()
+
     def _pack_head(self, sd):
         import torch
         dev = self.device
         z = {}
-
-        def W(key, rows=None, cols=None):      # 1x1 conv / linear weight -> fp16 [rows, cols] (zero padded)
-            t = sd[key + '.weight'].detach().to(dev).float()
-            t = t.reshape(t.shape[0], -1)
-            r, c = rows or t.shape[0], cols or t.shape[1]
-            o = torch.zeros(r, c, dtype=torch.float16, device=dev)
-            o[:t.shape[0], :t.shape[1]] = t.to(torch.float16)
-            return o
-
-        def Bv(key, n=None):
-            t = sd[key + '.bias'].detach().to(dev).float().reshape(-1)
-            o = torch.zeros(n or t.numel(), dtype=torch.float32, device=dev)
-            o[:t.numel()] = t
-            return o
-
+        W = lambda key, rows=None, cols=None: self._hw(sd, key, rows, cols)
+        Bv = lambda key, n=None: self._hb(sd, key, n)
         z['conv2'] = (W('conv2'), Bv('conv2'))
         z['emb'] = (W('patch_transformer.embedding_convPxP'), Bv('patch_transformer.embedding_convPxP'))
         layers = []
@@ -1157,10 +1168,7 @@ class ZoeDepthNKEngine(DptBeitEngine):
             w2c[k] = sd[f'conditional_log_binomial.{n}.mlp.2.weight'].detach().to(dev).float().reshape(4, 40)
             b2c[k] = sd[f'conditional_log_binomial.{n}.mlp.2.bias'].detach().to(dev).float()
         z['clb'] = (we, wo.contiguous(), b0.contiguous(), w2c.contiguous(), b2c.contiguous())
-        # out_conv with 64 output channels (32 real + 32 zero) so the stored activation is a valid GEMM-friendly NHWC tensor
-        h = 'depth_head.'
-        z['oc2_w'] = _conv_w(self._oc2_weight.to(dev), self.F2p, 32)
-        z['oc2_b'] = self._oc2_bias.to(dev).float().contiguous()
+        self._pack_out_conv(z)
         self.z = z
         self._pe_cache = {}
 
@@ -1182,38 +1190,56 @@ class ZoeDepthNKEngine(DptBeitEngine):
         return self._pe_cache[S]
 
     def _zbuffers(self, F, nh, nw, b):
+        """Head buffers; the widths follow the packed weights (NK: two heads side by side; N / K: one head)."""
         import torch
         key = (F, nh, nw)
         if self._zbuf_key == key:
             return self._zbufs
-        dev = self.device
+        dev, z = self.device, self.z
         h16 = lambda *s: torch.empty(*s, dtype=torch.float16, device=dev)
         f32 = lambda *s: torch.empty(*s, dtype=torch.float32, device=dev)
         s3 = b['sizes'][3]
         n0 = s3[0] * s3[1]
         S = n0 + 1
         levels = list(b['up_sizes'])                       # (h, w) of refinenet4..1 outputs
-        zb = dict(x16=h16(F * n0, self.Fp), emb=h16(F * n0, 128), X=f32(F * S, 128), h=h16(F * S, 128), qkv=h16(F * S, 384), att=h16(F * S, 128),
-                  ff=h16(F * S, 1024), c1=h16(F, 128), logits=f32(F, 32), s0=h16(F * n0, 128), seed=f32(F * n0, 128), bprev=f32(F * n0, 64),
-                  p0=h16(F * n0, 64), pemb=h16(F * n0, 128), S=S, n0=n0, levels=levels)
-        zb['t'] = [h16(F * h * w, 64) for h, w in levels]
+        ph = z['sproj'][0][0].shape[0]                      # projector hidden width
+        aw, an = z['att'][0][0][0].shape[0], z['att'][0][1][0].shape[0]     # attractor hidden width, attractor GEMM output width
+        zb = dict(x16=h16(F * n0, self.Fp), s0=h16(F * n0, z['seed0'][0].shape[0]), seed=f32(F * n0, z['seed2'][0].shape[0]),
+                  bprev=f32(F * n0, 64), p0=h16(F * n0, ph), pemb=h16(F * n0, 128), S=S, n0=n0, levels=levels)
+        if 'layers' in z:                                  # the router of ZoeDepth-NK
+            zb.update(emb=h16(F * n0, 128), X=f32(F * S, 128), h=h16(F * S, 128), qkv=h16(F * S, 384), att=h16(F * S, 128),
+                      ff=h16(F * S, 1024), c1=h16(F, 128), logits=f32(F, 32))
+        zb['t'] = [h16(F * h * w, ph) for h, w in levels]
         zb['bemb'] = [h16(F * h * w, 128) for h, w in levels]
         zb['xin'] = [h16(F * h * w, 128) for h, w in levels]
-        zb['a0'] = [h16(F * h * w, 256) for h, w in levels]
-        zb['A'] = [f32(F * h * w, 64) for h, w in levels]
+        zb['a0'] = [h16(F * h * w, aw) for h, w in levels]
+        zb['A'] = [f32(F * h * w, an) for h, w in levels]
         zb['bnew'] = [f32(F * h * w, 64) for h, w in levels]
         zb['ze'] = f32(F * levels[3][0] * levels[3][1], 128)
         zb['o32'] = h16(F, nh, nw, 32)
         zb['d'] = f32(F, nh, nw)
+        self._extra_zbuffers(zb, F, levels)
         self._zbufs, self._zbuf_key = zb, key
         return zb
 
+    def _extra_zbuffers(self, zb, F, levels):
+        pass
+
     # ---- forward -------------------------------------------------------------------------------------------------------
+    def _lin(self, a, lda, wb, M, N, K, out=None, ldc=None, act=_lib.ACT_NONE, f32out=None, resid=None):
+        wt, bias = wb
+        if resid is not None:
+            self.ops.gemm(a, lda, wt, K, M, N, K, epi=_lib.EPI_RESID_F32, bias=bias, X=resid, ldx=N, gamma=self.z['ones128'])
+        elif f32out is not None:
+            self.ops.gemm(a, lda, wt, K, M, N, K, epi=_lib.EPI_STORE_F32, act=act, bias=bias, X=f32out, ldx=N)
+        else:
+            self.ops.gemm(a, lda, wt, K, M, N, K, act=act, bias=bias, C=out, ldc=ldc or N)
+
     def forward_batch(self, rgb, net_w, net_h=None, out_hw=None):
         """rgb: uint8 CUDA [B,H,W,3] -> float32 CUDA [B,H,W] metric depth (what estimatezoedepth returns; invert = True)."""
         import torch
         L = self.ops.L
-        ops, z = self.ops, self.z
+        ops = self.ops
         st = _lib.stream_ptr
         B, H, W, _ = rgb.shape
         net_h = net_h if net_h is not None else net_w
@@ -1228,28 +1254,56 @@ class ZoeDepthNKEngine(DptBeitEngine):
         self.run_network(b, F, nh, nw)
         zb = self._zbuffers(F, nh, nw, b)
         Fp = self.Fp
-        E_, A_ = _lib, _lib
         # out_conv activation (MidasCore hooks output_conv[3], the 32-channel ReLU)
         t = b['up_sizes'][3]
         ops.conv3x3(b['path'][3], F, t[0], t[1], Fp, self.w['oc1_w'], self.F2p, bias=self.w['oc1_b'], C=b['oc1'])
         ops.resize_nhwc(b['oc1'], F, t[0], t[1], self.F2p, b['oc1u'], nh, nw)
-        ops.conv3x3(b['oc1u'], F, nh, nw, self.F2p, z['oc2_w'], 32, act=A_.ACT_RELU, bias=z['oc2_b'], C=zb['o32'])
+        ops.conv3x3(b['oc1u'], F, nh, nw, self.F2p, self.z['oc2_w'], 32, act=_lib.ACT_RELU, bias=self.z['oc2_b'], C=zb['o32'])
+        # x = conv2(bottleneck) (zoedepth_nk_v1.py:176-178, zoedepth_v1.py:145-146)
+        self._lin(b['l'][3], Fp, self.z['conv2'], F * zb['n0'], Fp, Fp, out=zb['x16'])
+        self._metric_head(b, zb, F, nh, nw)                 # -> zb['d'], metric depth per forward at the net size
+        # un-pad / un-flip / average (depth_model.py:88-129)
+        out = torch.empty(B, H, W, dtype=torch.float32, device=self.device)
+        _lib.check(L.dm_zoe_tta_combine(zb['d'].data_ptr(), B, nh, nw, pad_h, pad_w, H, W, out.data_ptr(), st()), "dm_zoe_tta_combine")
+        ops.launches += 1
+        return out
+
+    def _seed_embedding(self, zb, F):
+        """seed projector (zoedepth_nk_v1.py:206, zoedepth_v1.py:153)"""
+        n0, z, ph = zb['n0'], self.z, zb['p0'].shape[1]
+        self._lin(zb['x16'], self.Fp, z['sproj'][0], F * n0, ph, self.Fp, out=zb['p0'], act=_lib.ACT_RELU)
+        self._lin(zb['p0'], ph, z['sproj'][1], F * n0, 128, ph, out=zb['pemb'])
+
+    def _attractor_levels(self, b, zb, F, attract):
+        """the four projector + attractor levels (zoedepth_nk_v1.py:207-214, zoedepth_v1.py:156-161).  attract(i, A, b_prev, hp,
+        wp, h, w) runs level i's attractor kernel from the GEMM output A, writing zb['bnew'][i].  Returns the last level's size."""
+        z, Fp = self.z, self.Fp
+        L = self.ops.L
+        bprev, pemb, (hp, wp) = zb['bprev'], zb['pemb'], b['sizes'][3]
+        ph = zb['t'][0].shape[1]
+        for i, (h, w) in enumerate(zb['levels']):
+            M = F * h * w
+            aw, an = z['att'][i][0][0].shape[0], z['att'][i][1][0].shape[0]
+            self._lin(b['path'][i], Fp, z['proj'][i][0], M, ph, Fp, out=zb['t'][i], act=_lib.ACT_RELU)
+            self._lin(zb['t'][i], ph, z['proj'][i][1], M, 128, ph, out=zb['bemb'][i])
+            _lib.check(L.dm_resize_add_nhwc_f16(zb['bemb'][i].data_ptr(), pemb.data_ptr(), F, hp, wp, 128, zb['xin'][i].data_ptr(), h, w,
+                                                _lib.stream_ptr()), "dm_resize_add_nhwc_f16")
+            self._lin(zb['xin'][i], 128, z['att'][i][0], M, aw, 128, out=zb['a0'][i], act=_lib.ACT_RELU)
+            self._lin(zb['a0'][i], aw, z['att'][i][1], M, an, aw, f32out=zb['A'][i])
+            attract(i, zb['A'][i], bprev, hp, wp, h, w)
+            self.ops.launches += 2
+            bprev, pemb, (hp, wp) = zb['bnew'][i], zb['bemb'][i], (h, w)
+        return hp, wp
+
+    def _metric_head(self, b, zb, F, nh, nw):
+        L = self.ops.L
+        ops, z = self.ops, self.z
+        st = _lib.stream_ptr
+        E_, A_ = _lib, _lib
         n0, S = zb['n0'], zb['S']
-        s3 = b['sizes'][3]
-
-        def lin(a, lda, wb, M, N, K, out=None, ldc=None, act=A_.ACT_NONE, f32out=None, resid=None):
-            wt, bias = wb
-            if resid is not None:
-                ops.gemm(a, lda, wt, K, M, N, K, epi=E_.EPI_RESID_F32, bias=bias, X=resid, ldx=N, gamma=z['ones128'])
-            elif f32out is not None:
-                ops.gemm(a, lda, wt, K, M, N, K, epi=E_.EPI_STORE_F32, act=act, bias=bias, X=f32out, ldx=N)
-            else:
-                ops.gemm(a, lda, wt, K, M, N, K, act=act, bias=bias, C=out, ldc=ldc or N)
-
-        # x = conv2(bottleneck) (zoedepth_nk_v1.py:176-178)
-        lin(b['l'][3], Fp, z['conv2'], F * n0, Fp, Fp, out=zb['x16'])
+        lin = self._lin
         # ---- router: PatchTransformerEncoder (patch size 1) + MLP classifier (:186-195) ----
-        lin(zb['x16'], Fp, z['emb'], F * n0, 128, Fp, out=zb['emb'])
+        lin(zb['x16'], self.Fp, z['emb'], F * n0, 128, self.Fp, out=zb['emb'])
         ops.tokens(zb['emb'], z['zeros128'], self._router_pe(S), zb['X'], F, n0, 128)
         _lib.check(L.dm_cast_f32_f16(zb['X'].data_ptr(), F * S * 128, zb['h'].data_ptr(), st()), "dm_cast_f32_f16")
         ops.launches += 1
@@ -1269,36 +1323,148 @@ class ZoeDepthNKEngine(DptBeitEngine):
         lin(zb['c1'], 128, z['cls2'], F, 32, 128, f32out=zb['logits'])
         lg = zb['logits']
         # ---- seed bins + seed embedding (:197-206) ----
-        lin(zb['x16'], Fp, z['seed0'], F * n0, 128, Fp, out=zb['s0'], act=A_.ACT_RELU)
+        lin(zb['x16'], self.Fp, z['seed0'], F * n0, 128, self.Fp, out=zb['s0'], act=A_.ACT_RELU)
         lin(zb['s0'], 128, z['seed2'], F * n0, 128, 128, f32out=zb['seed'])
         _lib.check(L.dm_zoe_select_softplus(zb['seed'].data_ptr(), 128, lg.data_ptr(), 32, F, n0, zb['bprev'].data_ptr(), st()), "dm_zoe_select_softplus")
-        lin(zb['x16'], Fp, z['sproj'][0], F * n0, 64, Fp, out=zb['p0'], act=A_.ACT_RELU)
-        lin(zb['p0'], 64, z['sproj'][1], F * n0, 128, 64, out=zb['pemb'])
+        self._seed_embedding(zb, F)
         ops.launches += 1
         # ---- attractor levels (:207-214) ----
-        bprev, pemb, (hp, wp) = zb['bprev'], zb['pemb'], s3
-        for i, (h, w) in enumerate(zb['levels']):
-            M = F * h * w
-            lin(b['path'][i], Fp, z['proj'][i][0], M, 64, Fp, out=zb['t'][i], act=A_.ACT_RELU)
-            lin(zb['t'][i], 64, z['proj'][i][1], M, 128, 64, out=zb['bemb'][i])
-            _lib.check(L.dm_resize_add_nhwc_f16(zb['bemb'][i].data_ptr(), pemb.data_ptr(), F, hp, wp, 128, zb['xin'][i].data_ptr(), h, w, st()),
-                       "dm_resize_add_nhwc_f16")
-            lin(zb['xin'][i], 128, z['att'][i][0], M, 256, 128, out=zb['a0'][i], act=A_.ACT_RELU)
-            lin(zb['a0'][i], 256, z['att'][i][1], M, 64, 256, f32out=zb['A'][i])
-            _lib.check(L.dm_zoe_attractor(zb['A'][i].data_ptr(), 64, lg.data_ptr(), 32, bprev.data_ptr(), F, hp, wp, h, w, zb['bnew'][i].data_ptr(), st()),
+        def attract(i, A, bprev, hp, wp, h, w):
+            _lib.check(L.dm_zoe_attractor(A.data_ptr(), 64, lg.data_ptr(), 32, bprev.data_ptr(), F, hp, wp, h, w, zb['bnew'][i].data_ptr(), st()),
                        "dm_zoe_attractor")
-            ops.launches += 2
-            bprev, pemb, (hp, wp) = zb['bnew'][i], zb['bemb'][i], (h, w)
-        # ---- conditional log-binomial + expectation (:216-236), then un-pad / un-flip / average (depth_model.py:88-129) ----
+        hp, wp = self._attractor_levels(b, zb, F, attract)
+        bprev = zb['bnew'][3]
+        # ---- conditional log-binomial + expectation (:216-236) ----
         we, wo, b0, w2c, b2c = z['clb']
         ops.gemm(zb['bemb'][3], 128, we, 128, F * hp * wp, 128, 128, epi=E_.EPI_STORE_F32, X=zb['ze'], ldx=128)
         _lib.check(L.dm_zoe_clb_final(zb['o32'].data_ptr(), 32, zb['ze'].data_ptr(), 128, bprev.data_ptr(), lg.data_ptr(), 32, wo.data_ptr(), b0.data_ptr(),
                                       w2c.data_ptr(), b2c.data_ptr(), F, nh, nw, hp, wp, ZOE_CONFIG['min_temp'], ZOE_CONFIG['max_temp'],
                                       zb['d'].data_ptr(), st()), "dm_zoe_clb_final")
-        out = torch.empty(B, H, W, dtype=torch.float32, device=self.device)
-        _lib.check(L.dm_zoe_tta_combine(zb['d'].data_ptr(), B, nh, nw, pad_h, pad_w, H, W, out.data_ptr(), st()), "dm_zoe_tta_combine")
-        ops.launches += 2
-        return out
+        ops.launches += 1
+
+
+# ZoeDepth-N / -K as the reference builds them: get_config("zoedepth", "infer"[, config_version="kitti"]) -> ZoeDepth(core, **config)
+# (src/depthmap_generation.py:196-205, dzoedepth/models/zoedepth/config_zoedepth*.json).  min / max depth are the constructor's
+# defaults for BOTH (infer mode merges no dataset config, so K does not get KITTI's 80); the attractor counts are passed by keyword,
+# so the levels really have 16, 8, 4, 1 attractors.
+ZOE_SINGLE = {7: dict(name='zoedepth_n', normed=False, n_attractors=(16, 8, 4, 1), min_depth=1e-3, max_depth=10.0),
+              8: dict(name='zoedepth_k', normed=True, n_attractors=(16, 8, 4, 1), min_depth=1e-3, max_depth=10.0)}
+
+
+class ZoeDepthEngine(ZoeDepthNKEngine):
+    """ZoeDepth-N (model type 7) and ZoeDepth-K (type 8): the single metric head of ZoeDepth.forward
+    (zoedepth/zoedepth_v1.py:120-186) on the core, pre-processing and pad + flip TTA of ZoeDepthNKEngine.  No router.
+      N: softplus bin centres (SeedBinRegressorUnnormed + AttractorLayerUnnormed).
+      K: normed bin centres (SeedBinRegressor + AttractorLayer): widths normalised over the 64 bins and accumulated into
+         centres in [min, max]; each attractor level sorts and clips the scaled centres, the next level gets the unsorted
+         normed ones.
+    The log-binomial MLP also sees the core's own relative depth, relu(output_conv.4(out_conv)), as a 33rd input channel.
+    A missing or mis-shaped head weight raises ValueError naming the key."""
+
+    def __init__(self, state_dict, model_type, device, core_name='beitl16_384'):
+        if model_type not in ZOE_SINGLE:
+            raise ValueError(f"ZoeDepthEngine builds model types 7 (ZoeDepth-N) and 8 (ZoeDepth-K), not {model_type}")
+        self.model_type = model_type
+        self.zconf = ZOE_SINGLE[model_type]
+        super().__init__(state_dict, device, core_name)
+
+    def _pack(self, sd):
+        for k, shape in (('scratch.output_conv.4.weight', (1, 32, 1, 1)), ('scratch.output_conv.4.bias', (1,))):
+            if k not in sd:
+                raise ValueError(f"ZoeDepth checkpoint: core.core.{k} is missing")
+            if tuple(sd[k].shape) != shape:
+                raise ValueError(f"ZoeDepth checkpoint: core.core.{k} has shape {tuple(sd[k].shape)}, expected {shape}")
+        self._rel_w = sd['scratch.output_conv.4.weight'].detach().float().reshape(32)
+        self._rel_b = float(sd['scratch.output_conv.4.bias'].detach().float().reshape(-1)[0])
+        super()._pack(sd)
+
+    def head_shapes(self):
+        """{key: (out, in)} of every 1x1 conv of the single head (weights [out, in, 1, 1], biases [out])."""
+        feat, emb, nb = self.cfg['features'], 128, 64
+        per = 2 if self.zconf['normed'] else 1
+        s = {'conv2': (feat, feat), 'seed_bin_regressor._net.0': (256, feat), 'seed_bin_regressor._net.2': (nb, 256),
+             'seed_projector._net.0': (128, feat), 'seed_projector._net.2': (emb, 128),
+             'conditional_log_binomial.mlp.0': ((33 + emb) // 2, 33 + emb), 'conditional_log_binomial.mlp.2': (4, (33 + emb) // 2)}
+        for i, n in enumerate(self.zconf['n_attractors']):
+            s[f'projectors.{i}._net.0'] = (128, feat)
+            s[f'projectors.{i}._net.2'] = (emb, 128)
+            s[f'attractors.{i}._net.0'] = (128, emb)
+            s[f'attractors.{i}._net.2'] = (per * n, 128)
+        return s
+
+    def _pack_head(self, sd):
+        import torch
+        dev = self.device
+        for key, (o, i) in self.head_shapes().items():
+            for suffix, shape in (('.weight', (o, i, 1, 1)), ('.bias', (o,))):
+                if key + suffix not in sd:
+                    raise ValueError(f"ZoeDepth checkpoint: {key + suffix} is missing")
+                if tuple(sd[key + suffix].shape) != shape:
+                    raise ValueError(f"ZoeDepth checkpoint: {key + suffix} has shape {tuple(sd[key + suffix].shape)}, expected {shape}")
+        z = {}
+        W = lambda key, rows=None, cols=None: self._hw(sd, key, rows, cols)
+        Bv = lambda key, n=None: self._hb(sd, key, n)
+        z['ones128'] = torch.ones(128, dtype=torch.float32, device=dev)
+        z['conv2'] = (W('conv2'), Bv('conv2'))
+        z['seed0'] = (W('seed_bin_regressor._net.0'), Bv('seed_bin_regressor._net.0'))
+        z['seed2'] = (W('seed_bin_regressor._net.2'), Bv('seed_bin_regressor._net.2'))
+        z['sproj'] = ((W('seed_projector._net.0'), Bv('seed_projector._net.0')), (W('seed_projector._net.2'), Bv('seed_projector._net.2')))
+        z['proj'] = [((W(f'projectors.{i}._net.0'), Bv(f'projectors.{i}._net.0')), (W(f'projectors.{i}._net.2'), Bv(f'projectors.{i}._net.2'))) for i in range(4)]
+        # attractor GEMM output padded to 32 columns (N: n softplus inputs, K: 2n ReLU inputs of which the even ones are used)
+        z['att'] = [((W(f'attractors.{i}._net.0'), Bv(f'attractors.{i}._net.0')), (W(f'attractors.{i}._net.2', rows=32), Bv(f'attractors.{i}._net.2', 32)))
+                    for i in range(4)]
+        # conditional log-binomial: mlp.0 [80, 161] split into out_conv (32), relative depth (1) and bin embedding (128) columns;
+        # the last part is a GEMM before the up-sampling, as for NK
+        m0 = sd['conditional_log_binomial.mlp.0.weight'].detach().to(dev).float().reshape(80, 161)
+        we = torch.zeros(128, 128, dtype=torch.float16, device=dev)
+        we[:80] = m0[:, 33:].to(torch.float16)
+        f32 = lambda t: t.detach().to(dev).float().contiguous()
+        z['clb'] = (we, f32(m0[:, :32].t()), f32(m0[:, 32]), f32(sd['conditional_log_binomial.mlp.0.bias']),
+                    f32(sd['conditional_log_binomial.mlp.2.weight'].reshape(4, 80)), f32(sd['conditional_log_binomial.mlp.2.bias']))
+        z['rel'] = (self._rel_w.to(dev).contiguous(), self._rel_b)
+        self._pack_out_conv(z)
+        self.z = z
+
+    def _extra_zbuffers(self, zb, F, levels):
+        import torch
+        if self.zconf['normed']:
+            h, w = levels[3]
+            zb['Bc'] = torch.empty(F * h * w, 64, dtype=torch.float32, device=self.device)    # sorted, clipped centres of the last level
+        else:
+            zb['head0'] = torch.zeros(F, 2, dtype=torch.float32, device=self.device)          # select_softplus with head 0 for every forward
+
+    def _metric_head(self, b, zb, F, nh, nw):
+        L = self.ops.L
+        ops, z, c = self.ops, self.z, self.zconf
+        st = _lib.stream_ptr
+        n0, Fp = zb['n0'], self.Fp
+        mn, mx = c['min_depth'], c['max_depth']
+        # ---- seed bins (zoedepth_v1.py:147-151) + seed embedding ----
+        s0w, nb = z['seed0'][0].shape[0], z['seed2'][0].shape[0]
+        self._lin(zb['x16'], Fp, z['seed0'], F * n0, s0w, Fp, out=zb['s0'], act=_lib.ACT_RELU)
+        self._lin(zb['s0'], s0w, z['seed2'], F * n0, nb, s0w, f32out=zb['seed'])
+        if c['normed']:
+            _lib.check(L.dm_zoe_seed_normed(zb['seed'].data_ptr(), nb, F * n0, mn, mx, zb['bprev'].data_ptr(), st()), "dm_zoe_seed_normed")
+        else:
+            _lib.check(L.dm_zoe_select_softplus(zb['seed'].data_ptr(), nb, zb['head0'].data_ptr(), 2, F, n0, zb['bprev'].data_ptr(), st()),
+                       "dm_zoe_select_softplus")
+        ops.launches += 1
+        self._seed_embedding(zb, F)
+
+        # ---- attractor levels (:156-161) ----
+        def attract(i, A, bprev, hp, wp, h, w):
+            Bs = zb['Bc'].data_ptr() if (c['normed'] and i == 3) else None
+            _lib.check(L.dm_zoe_attractor_single(A.data_ptr(), A.shape[1], c['n_attractors'][i], int(c['normed']), bprev.data_ptr(), F, hp, wp, h, w,
+                                                 mn, mx, zb['bnew'][i].data_ptr(), Bs, st()), "dm_zoe_attractor_single")
+        hp, wp = self._attractor_levels(b, zb, F, attract)
+        centres = zb['Bc'] if c['normed'] else zb['bnew'][3]
+        # ---- conditional log-binomial on cat(out_conv, rel_depth, b_emb) + expectation (:163-186) ----
+        we, wo, wr, b0, w2c, b2c = z['clb']
+        ops.gemm(zb['bemb'][3], 128, we, 128, F * hp * wp, 128, 128, epi=_lib.EPI_STORE_F32, X=zb['ze'], ldx=128)
+        _lib.check(L.dm_zoe_clb_final_single(zb['o32'].data_ptr(), 32, zb['ze'].data_ptr(), 128, centres.data_ptr(), wo.data_ptr(), wr.data_ptr(),
+                                             b0.data_ptr(), w2c.data_ptr(), b2c.data_ptr(), z['rel'][0].data_ptr(), z['rel'][1], F, nh, nw, hp, wp,
+                                             ZOE_CONFIG['min_temp'], ZOE_CONFIG['max_temp'], zb['d'].data_ptr(), st()), "dm_zoe_clb_final_single")
+        ops.launches += 1
 
 
 class ModelHolder:
@@ -1402,20 +1568,24 @@ class ModelHolder:
                 if "optimizer" in sd:
                     sd = sd["model"]
             model = NativeDepthModel(sd, model_type, torch.device(device))
-        elif model_type == 9:  # zoedepth_nk (src/depthmap_generation.py:221-226: ZoeD_M12_NK.pt)
+        elif model_type in (7, 8, 9):  # zoedepth_n / _k / _nk (src/depthmap_generation.py:196-226: ZoeD_M12_N.pt / _K.pt / _NK.pt)
             if self.weights_provider is not None:
                 sd = self.weights_provider(model_type)
             else:
-                model_path = "./models/zoedepth/ZoeD_M12_NK.pt"
+                model_path = "./models/zoedepth/" + {7: "ZoeD_M12_N.pt", 8: "ZoeD_M12_K.pt", 9: "ZoeD_M12_NK.pt"}[model_type]
                 if not os.path.exists(model_path):
                     raise FileNotFoundError(f"{model_path} not found (depthmap_b200 does not download checkpoints)")
                 sd = torch.load(model_path, map_location='cpu')
                 if "model" in sd:           # dzoedepth/models/model_io.py:52-53
                     sd = sd["model"]
-            model = ZoeDepthNKEngine(sd, torch.device(device))
+            if model_type == 9:
+                model = ZoeDepthNKEngine(sd, torch.device(device))
+            else:
+                model = ZoeDepthEngine(sd, model_type, torch.device(device))
         else:
             raise NotImplementedError(f"model_type {model_type} is not implemented in depthmap_b200 yet "
-                                      f"(implemented: 0 = LeReS res101; 1, 2 = DPT-BEiT-L 512/384; 3 = DPT-Large 384; 9 = ZoeDepth-NK; 12, 13, 14 = Depth-Anything-V2 S/B/L)")
+                                      f"(implemented: 0 = LeReS res101; 1, 2 = DPT-BEiT-L 512/384; 3 = DPT-Large 384; 7, 8, 9 = ZoeDepth-N/K/NK; "
+                                      f"12, 13, 14 = Depth-Anything-V2 S/B/L)")
         self.depth_model = model
         self.depth_model_type = model_type
         self.resize_mode = "minimal"
@@ -1470,7 +1640,7 @@ class ModelHolder:
             import torch
             preds = [self.pix2pix_model.run(rgb[i].cpu().numpy(), self.boost_rmax, to_host=False) for i in range(rgb.shape[0])]
             return torch.stack(preds), self.depth_model_type in [0, 7, 8, 9, 10]
-        if self.depth_model_type in (0, 1, 2, 3, 9, 12, 13, 14):
+        if self.depth_model_type in (0, 1, 2, 3, 7, 8, 9, 12, 13, 14):
             pred = self.depth_model.forward_batch(rgb, net_width, net_height)
         else:
             raise NotImplementedError(f"model_type {self.depth_model_type}")
